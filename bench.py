@@ -2,6 +2,7 @@
 """Benchmark of the shapegan hot path on B200 (contract: see the task statement / DESIGN.md "Measurement").
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload wgan_gp|wgan|gan|hybrid|autodecoder]
+                    [--dump-outputs DIR]
 
 One "step" of the default workload = BASELINE.json configs[1]: the 3D-CNN WGAN-GP G+D step on 32^3 voxels, batch 64 per GPU,
 bf16 -- train_wgan.py:62-71 (critic update: fake B + real B, RMSprop) with the gradient penalty of
@@ -19,6 +20,10 @@ train_hybrid_progressive_gan.py:102-111 in place of the weight clip (SURVEY D1; 
   sdfnet    : SDFNet Mpoints/s (fused forward, configs[2] autodecoder step)
   cpu_baseline : the oracle port of the same step (oracle/ref_steps.py, torch CPU fp32 = what the reference runs on a CPU host)
               timed on this box's cores
+
+--dump-outputs DIR writes what the timed step returned in its last timed iteration -- its loss scalars and the updated parameters
+and buffers of the models it trains -- as DIR/<name>.npy (float32).  The inputs and initial weights are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -269,13 +274,12 @@ def cpu_step(workload, b, ad_shapes=8):
 
 def run_reference(args, rank, world):
     """The reference's own CPU implementation of the step (oracle port), on the host threads that run it fastest, at the GPU arm's
-    config (same per-GPU batch; EXACTLY --steps timed steps unless that would exceed ~150 s, which is then stated)."""
+    config (same per-GPU batch; exactly --steps timed steps)."""
     if rank != 0:
         return
     run, units, unit, metric, sample = cpu_step(args.workload, args.batch)
     cores, t_one, calib = pick_cpu_threads(run)
-    budget = 150.0
-    steps = max(1, min(args.steps, int(budget / max(t_one, 1e-3))))
+    steps = args.steps
     warm = max(0, min(args.warmup, int(30.0 / max(t_one, 1e-3))))
     for _ in range(warm):
         run()
@@ -439,6 +443,31 @@ class Workload:
         self.h_loss = torch.zeros(d_loss.numel()).pin_memory()
 
 
+def model_state(prefix, module):
+    """{prefix.name: tensor} of the parameters and floating-point buffers of a module (aliased parameters once)"""
+    out = {'%s.%s' % (prefix, k): v for k, v in module.named_parameters()}
+    out.update({'%s.%s' % (prefix, k): v for k, v in module.named_buffers() if v.is_floating_point()})
+    return out
+
+
+def named_losses(d_loss, names):
+    return {n: d_loss[i] for i, n in enumerate(names)}
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in float32"""
+    import numpy as np
+    total = sum(t.numel() * 4 for t in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit('bench.py: --dump-outputs would write %d bytes (limit %d)' % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def make_cnn_workload(kind, b, rank, world, dev, gp_fused=True):
     """wgan / wgan_gp / gan on gan.Generator + gan.Discriminator (random-init weights of the reference architecture)."""
     from model.gan import Discriminator, Generator
@@ -468,6 +497,8 @@ def make_cnn_workload(kind, b, rank, world, dev, gp_fused=True):
     nec, written = gflop_per_sample(kind)
     w = Workload(kind, body, host, devt, d_loss, b * VOX, nec * b, written * b)
     w.keep = (gen, dis, step)
+    losses = ('generator_loss', 'fake_loss', 'valid_loss') if kind == 'gan' else ('critic_loss', 'generator_loss')
+    w.outputs = {**named_losses(d_loss, losses), **model_state('generator', gen), **model_state('critic', dis)}
     w.dp_note = (step.copt if kind != 'gan' else step.dopt).dp_note
     return w
 
@@ -496,6 +527,8 @@ def make_hybrid_workloads(b, rank, world, dev):
     wd = Workload('hybrid_d_update', d_body, host, devt, dl, b * 64 ** 3, d_nec * b)
     wg = Workload('hybrid_g_update', g_body, [host[1]], [devt[1]], gl, b * 64 ** 3, g_nec * b)
     wd.keep = wg.keep = (gen, dis, step)
+    wd.outputs = {**named_losses(dl, ('critic_loss', 'gradient_penalty')), **named_losses(gl, ('generator_loss',)),
+                  **model_state('generator', gen), **model_state('critic', dis)}
     wd.dp_note = wg.dp_note = step.dopt.dp_note
     return wd, wg
 
@@ -638,7 +671,12 @@ def main():
     ap.add_argument('--no-extra', action='store_true', help='skip the sub-blocks of the other BASELINE configs')
     ap.add_argument('--extra-steps', type=int, default=10)
     ap.add_argument('--ad-shapes', type=int, default=512, help='autodecoder workload: number of shapes (16384 points each)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs applies to the B200 arm')
     if args.batch is None:
         args.batch = {'gan': 32, 'hybrid': 2}.get(args.workload, 64)
     if args.impl == 'reference':
@@ -668,11 +706,14 @@ def main():
         res = measure(wd, args.steps, args.warmup, world, flush, lib, args.no_graph, sampler)
         res_g = measure(wg, max(3, args.steps // 5), 3, world, flush, lib, args.no_graph)
         metric = 'hybrid_it3_d_update_voxels_per_s'
+        w = wd
     else:
         w = make_cnn_workload(args.workload, b, rank, world, dev)
         res = measure(w, args.steps, args.warmup, world, flush, lib, args.no_graph, sampler)
         res_g = None
         metric = 'wgan_gd_step_voxels_per_s' if args.workload.startswith('wgan') else 'gan_iteration_voxels_per_s'
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, w.outputs)
     clocks = sampler.finish() if sampler is not None else None
     extras = None if args.no_extra else extra_configs(args, rank, world, dev, flush, lib)
     err = lib.sg_check_device_error()
@@ -728,7 +769,7 @@ def bench_autodecoder(args, rank, world, dev, lib):
     torch.cuda.synchronize()
     barrier(world)
     total = 0.0
-    steps = min(args.steps, 10)
+    steps = args.steps
     for _ in range(steps):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); loss = step(pts, sdf, idx); e1.record()
@@ -737,6 +778,8 @@ def bench_autodecoder(args, rank, world, dev, lib):
     ms = max_over_ranks(total / steps, world)
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'loss': loss, 'latent_table': step.table, **model_state('sdf_net', net)})
     pk, src = peaks()
     tflops = 2.763e6 * n / (ms * 1e-3) / 1e12
     emit(json.dumps({

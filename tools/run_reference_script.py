@@ -6,7 +6,7 @@ and `itertools.count` capped so that the script's endless epoch loop ends after 
     python tools/run_reference_script.py /path/to/reference/train_wgan.py --epochs 1 --samples 96 -- nogui
 
 On a CUDA machine the script trains on libsg_b200; on a CPU-only host it runs up to its first forward pass, where the package
-raises its "no CPU fallback" error (tests/test_reference_scripts_cpu.py checks exactly that)."""
+raises its "no CPU fallback" error."""
 import argparse
 import itertools
 import os
